@@ -4,6 +4,7 @@
   python bench.py --gpus 1 --steps K --warmup W             native arm (libsdwalk.so)
   python bench.py --impl reference ...                       the reference's CPU path (oracle restatement), rank 0
   torchrun --nproc-per-node N bench.py --gpus N ...          one rank per GPU, frames sharded, NCCL gather
+  python bench.py ... --dump-outputs DIR                     also write the last timed step's frames to DIR/frames.npy
 
 Workload (config.workload): BASELINE.json configs[1] — SD-1.4 architecture, 512x512, fp16, PNDM 50 steps
 (51 UNet calls), classifier-free guidance 7.5, frames interpolated between 2 synthetic prompts; random-init weights
@@ -140,6 +141,23 @@ def cpu_reference_leg(steps, warmup, budget_s=150.0):
             "s_per_frame": spf, "t_unet_s": t_unet, "t_vae_s": t_vae, "steps_run": steps_run, "warmup_run": warm_run}
 
 
+DUMP_BYTES = 64_000_000  # at most this much in --dump-outputs DIR
+
+
+def dump_outputs(out_dir, frames):
+    """Write the uint8 frames [n, H, W, 3] a timed step returned as out_dir/frames.npy in float32.  When all n frames
+    exceed DUMP_BYTES, a fixed sample of whole frames is written: indices drawn without replacement by numpy's
+    default_rng(0), ascending.  Returns the indices written."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    x = frames.cpu().numpy()
+    n, keep = x.shape[0], (DUMP_BYTES - 128) // (x[0].size * 4)  # 128: the .npy header
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    np.save(os.path.join(out_dir, "frames.npy"), x[idx].astype(np.float32))
+    return idx
+
+
 def _stdout_to_stderr():
     """Route fd 1 to stderr while the benchmark runs: libraries (NCCL prints its version line from C) must not put
     anything on stdout next to the ONE JSON line."""
@@ -171,7 +189,11 @@ def main():
     ap.add_argument("--inference-steps", type=int, default=50)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frames of the last one to DIR/frames.npy (float32)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     saved_stdout = _stdout_to_stderr()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -254,7 +276,7 @@ def main():
         lat, emb = batch(i)
         u8 = eng.sample(lat, emb, unc, use_graph=not a.no_graph)
         if world > 1 and gather:
-            gather_frames(u8, F * world)  # decoded frames to rank 0 over NCCL
+            u8 = gather_frames(u8, F * world)  # decoded frames to rank 0 over NCCL (None on the other ranks)
         return u8
 
     for i in range(W):
@@ -267,7 +289,7 @@ def main():
     barrier()
     ev0.record()
     for i in range(K):
-        run_step(W + i)
+        out = run_step(W + i)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
@@ -276,6 +298,10 @@ def main():
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         ms = float(tt.item())
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        idx = dump_outputs(a.dump_outputs, out)
+        print(f"dump: frames {idx.tolist()} of {out.shape[0]} of timed step {K} -> "
+              f"{os.path.join(a.dump_outputs, 'frames.npy')}", file=sys.stderr)
     frames_total = K * F * world
     value = frames_total / (ms / 1e3)
 

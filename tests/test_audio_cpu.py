@@ -116,14 +116,18 @@ def test_package_entry_point_uses_the_restatement_without_librosa(tmp_path):
     assert T.shape == (60,) and abs(T[-1] - 1.0) < 1e-6 and (np.diff(T) > 0).all()
 
 
-def test_cfg5_schedule_fixture(audio):
+def test_cfg5_schedule_fixture(audio, tmp_path):
     """BASELINE configs[4]: T for the reference's own choice.wav with the example's arguments (fps 30, margin 1.0,
-    smooth 0.2) is committed as tests/golden/cfg5_choice_T.npy; where the reference checkout exists the restatement must
-    reproduce it, everywhere it must be a valid schedule (300 frames, in [0, 1], non-decreasing, ends at 1)."""
+    smooth 0.2) is committed as tests/golden/cfg5_choice_T.npy, the clip's PCM samples as tests/golden/cfg5_choice_wav.npz;
+    the restatement must reproduce T from that WAV, and T must be a valid schedule (300 frames, in [0, 1], non-decreasing,
+    ends at 1)."""
+    from scipy.io import wavfile
+
     T = np.load(os.path.join(ROOT, "tests", "golden", "cfg5_choice_T.npy"))
     assert T.shape == (300,) and T.dtype == np.float64
     assert T.min() >= 0.0 and abs(T[-1] - 1.0) < 1e-12 and np.all(np.diff(T) >= 0)
-    wav = "/root/reference/tests/samples/choice.wav"
-    if os.path.exists(wav):
-        again = audio.get_timesteps_arr(wav, offset=0, duration=10, fps=30, margin=1.0, smooth=0.2)
-        assert np.allclose(again, T, atol=1e-9)
+    clip = np.load(os.path.join(ROOT, "tests", "golden", "cfg5_choice_wav.npz"))
+    wav = tmp_path / "choice.wav"
+    wavfile.write(wav, int(clip["sr"]), clip["samples"])
+    again = audio.get_timesteps_arr(wav, offset=0, duration=10, fps=30, margin=1.0, smooth=0.2)
+    assert np.allclose(again, T, atol=1e-9)
