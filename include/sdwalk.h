@@ -184,12 +184,12 @@ typedef struct sdw_gemm_desc {
   int64_t ldc;
   int64_t o_sW, o_sH, o_sB;
   int32_t mode;              /* 0 plain, 1 GEGLU, 2 QKV with V^T scatter */
-  int32_t act;
+  int32_t act;               /* 0 none, 1 SiLU, 2 LeakyReLU(0.2) (applied after bias, before the residual) */
   float alpha;
   int32_t vt_col0, vt_d, vt_heads, vt_ntok;
   void* vt;
   int64_t vt_ld;
-  int32_t bn;                /* BLOCK_N: 0 auto, 64/128/160/256 */
+  int32_t bn;                /* BLOCK_N: 0 auto, 32/64/128/160/256 (32 and 64: one-CTA kernel only) */
   int32_t ver;               /* 0 auto, 1: one CTA per 128xBN tile, 2: persistent CTA pairs (256xBN) */
   int32_t nsub;              /* 0 auto, 1 / 2: accumulators per activation tile in the CTA-pair kernel */
   int32_t ew;                /* 0 auto, 2 / 4: epilogue warps per TMEM lane quarter of the CTA-pair kernel (4: needs the TMA epilogue) */
@@ -201,6 +201,9 @@ typedef struct sdw_gemm_desc {
 } sdw_gemm_desc;
 
 int sdw_gemm(const sdw_gemm_desc* desc, void* stream);
+/* the same GEMM with a second, scaled residual on the first residual's strides (plain mode, `resid` set):
+ * out = res2_scale * (epilogue result including resid) + resid2 — Real-ESRGAN's RRDB exit 0.2 * (0.2 * (acc + b) + x) + x0 */
+int sdw_gemm_res2(const sdw_gemm_desc* desc, const void* resid2, float res2_scale, void* stream);
 /* planner introspection, host only (also in plan-only mode): out = {kernel version, BLOCK_N, accumulators, epilogue warps
  * per lane quarter, tap reuse, TMA epilogue, pipeline stages, 0, grid size, tile w, tile h, tile b} */
 int sdw_debug_plan(const sdw_gemm_desc* desc, int32_t out[12]);
@@ -256,6 +259,38 @@ int sdw_clip_missing_params(const sdw_clip* e, const char** first_missing);
 /* ids: device int32 [B][max_positions] (token ids, already padded / truncated by the tokenizer);
  * out: device fp16 [B][max_positions][hidden] = last_hidden_state after the final LayerNorm */
 int sdw_clip_forward(sdw_clip* e, const int32_t* ids, int B, void* out_f16, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Real-ESRGAN 4x upsampler: replaces RealESRGANModel.forward (upsampling.py:30-55; basicsr RRDBNet x4plus under
+ * RealESRGANer.enhance with tile = 0, pre_pad = 0, outscale = 4) for `frames` frames per call.  Parameter names are
+ * basicsr's RRDBNet state-dict keys ("conv_first.weight", "body.{i}.rdb{1,2,3}.conv{1..5}.weight", "conv_body.*",
+ * "conv_up1.*", "conv_up2.*", "conv_hr.*", "conv_last.*"), handed over as fp16 in their own (OIHW / vector) layout.
+ * Life cycle as the CLIP tower: create -> arena_bytes -> bind(arena: caller-owned device memory, 4096-byte aligned; all
+ * launches are planned here) -> load_param x N -> forward x M -> destroy.
+ * ---------------------------------------------------------------------------------------- */
+typedef struct sdw_esrgan sdw_esrgan;
+typedef struct sdw_esrgan_config {
+  int32_t num_in_ch, num_out_ch;  /* 3, 3 */
+  int32_t num_feat, num_block, num_grow_ch;  /* 64, 23, 32 for RealESRGAN_x4plus */
+  int32_t scale;                  /* 4 only */
+  int32_t height, width;          /* input frame size */
+  int32_t frames;                 /* frames per forward call the activation buffers are sized for */
+} sdw_esrgan_config;
+int sdw_esrgan_create(const sdw_esrgan_config* cfg, sdw_esrgan** out);
+void sdw_esrgan_destroy(sdw_esrgan* e);
+int sdw_esrgan_arena_bytes(const sdw_esrgan* e, uint64_t* bytes);
+int sdw_esrgan_bind(sdw_esrgan* e, void* arena, uint64_t bytes);
+int sdw_esrgan_num_params(const sdw_esrgan* e);
+int sdw_esrgan_param_info(const sdw_esrgan* e, int index, const char** name, int64_t* numel);
+int sdw_esrgan_load_param(sdw_esrgan* e, const char* name, const void* src_f16, int64_t numel, void* stream);
+int sdw_esrgan_missing_params(const sdw_esrgan* e, const char** first_missing);
+/* in_u8 [n][H][W][3] RGB (n <= frames) -> out_u8 [n][4H][4W][3] = round(clamp(model(in / 255), 0, 1) * 255);
+ * out_f32 (optional): fp32 [n][4H][4W][3] model output before the clamp.  use_graph = 1 replays the whole forward as one
+ * CUDA graph (captured on first use per n; `stream` must then be a real stream, not the legacy default stream 0). */
+int sdw_esrgan_forward(sdw_esrgan* e, const uint8_t* in_u8, int n, uint8_t* out_u8, float* out_f32, int use_graph,
+                       void* stream);
+/* number of kernel launches (and copies) of one forward, as planned at bind */
+int sdw_esrgan_launches(const sdw_esrgan* e, int* n);
 
 /* ------------------------------------------------------------------------------------------
  * Frame-sharded walk over the GPUs of one box (one process per GPU): the three exchanges of the path, as thin NCCL

@@ -17,6 +17,7 @@ _LAZY = {
     "Engine": ("engine", "Engine"),
     "UNetConfig": ("configs", "UNetConfig"),
     "VAEConfig": ("configs", "VAEConfig"),
+    "RealESRGANModel": ("upsampling", "RealESRGANModel"),
 }
 
 

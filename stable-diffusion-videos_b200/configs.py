@@ -202,3 +202,66 @@ def random_state_dict(shapes: Dict[str, tuple], seed: int, dtype=None, device="c
             t = (torch.rand(shp, generator=g) * 2 - 1) * bound
         sd[name] = t.to(dtype or torch.float16).to(device)
     return sd
+
+
+@dataclass
+class ESRGANConfig:
+    """basicsr RRDBNet as RealESRGANModel builds it (the reference's upsampling.py:25): RealESRGAN_x4plus."""
+    num_in_ch: int = 3
+    num_out_ch: int = 3
+    num_feat: int = 64
+    num_block: int = 23
+    num_grow_ch: int = 32
+    scale: int = 4
+
+
+def esrgan_param_shapes(cfg: ESRGANConfig) -> Dict[str, tuple]:
+    """name -> shape of every RRDBNet parameter (basicsr state-dict keys, as in RealESRGAN_x4plus.pth)."""
+    o: Dict[str, tuple] = {}
+    nf, g = cfg.num_feat, cfg.num_grow_ch
+
+    def conv(name, cout, cin):
+        o[name + ".weight"] = (cout, cin, 3, 3)
+        o[name + ".bias"] = (cout,)
+
+    conv("conv_first", nf, cfg.num_in_ch)
+    for i in range(cfg.num_block):
+        for r in (1, 2, 3):
+            for k in range(4):
+                conv(f"body.{i}.rdb{r}.conv{k + 1}", g, nf + k * g)
+            conv(f"body.{i}.rdb{r}.conv5", nf, nf + 4 * g)
+    for name in ("conv_body", "conv_up1", "conv_up2", "conv_hr"):
+        conv(name, nf, nf)
+    conv("conv_last", cfg.num_out_ch, nf)
+    return o
+
+
+def esrgan_random_state_dict(cfg: ESRGANConfig, seed: int, dtype=None, device="cpu"):
+    """Random RRDBNet weights initialised as basicsr does: the dense-block convs get `default_init_weights(scale=0.1)`
+    (Kaiming-normal fan-in weights x 0.1, zero bias), every other conv torch's Conv2d default
+    (U(-1/sqrt(fan_in), 1/sqrt(fan_in)) for weight and bias).  Generated name-by-name in sorted order from one CPU
+    generator (deterministic).  One departure: `conv_last` gets half-scale weights and a bias of 0.5, so the untrained
+    model's image sits mid-range, as a trained model's does, instead of a third of its pixels clamping at 0 — parity
+    fixtures built on it then compare unsaturated pixels."""
+    import torch
+
+    shapes = esrgan_param_shapes(cfg)
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    sd = {}
+    for name in sorted(shapes):
+        shp = shapes[name]
+        wshp = shapes[name.rsplit(".", 1)[0] + ".weight"]
+        fan_in = wshp[1] * wshp[2] * wshp[3]
+        if name.startswith("body."):
+            if name.endswith("weight"):
+                t = torch.randn(shp, generator=g) * (2.0 / fan_in) ** 0.5 * 0.1
+            else:
+                t = torch.zeros(shp)
+        else:
+            t = (torch.rand(shp, generator=g) * 2 - 1) * fan_in ** -0.5
+            if name == "conv_last.weight":
+                t = t * 0.5
+            elif name == "conv_last.bias":
+                t = torch.full(shp, 0.5)
+        sd[name] = t.to(dtype or torch.float16).to(device)
+    return sd

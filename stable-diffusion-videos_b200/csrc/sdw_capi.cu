@@ -67,6 +67,17 @@ int sdw_gemm(const sdw_gemm_desc* c, void* stream) {
   return launch_gemm(L, static_cast<cudaStream_t>(stream));
 }
 
+int sdw_gemm_res2(const sdw_gemm_desc* c, const void* resid2, float res2_scale, void* stream) {
+  SDW_REQUIRE(c != nullptr && resid2 != nullptr, "null");
+  GemmDesc d;
+  if (int e = to_desc(c, d)) return e;
+  d.resid2 = static_cast<const __half*>(resid2);
+  d.res2_scale = res2_scale;
+  GemmLaunch L;
+  if (int e = plan_gemm(d, &L)) return e;
+  return launch_gemm(L, static_cast<cudaStream_t>(stream));
+}
+
 static int to_desc(const sdw_gemm_desc* c, GemmDesc& d) {
   d.A = static_cast<const __half*>(c->A);
   d.C = c->C; d.W = c->W; d.H = c->H; d.B = c->B;

@@ -166,6 +166,7 @@ int gemm_init() {
     return 2;
   }
   g_encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
+  if (int e = set_attr<32>()) return e;
   if (int e = set_attr<64>()) return e;
   if (int e = set_attr<128>()) return e;
   if (int e = set_attr<160>()) return e;
@@ -225,6 +226,8 @@ static int pow2_floor(int v) {
 int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
   SDW_REQUIRE(d.A && d.Wt && d.out, "null operand");
   SDW_REQUIRE(d.C > 0 && d.W > 0 && d.H > 0 && d.B > 0 && d.N > 0, "empty problem");
+  SDW_REQUIRE(d.act >= 0 && d.act <= 2, "act: 0 none, 1 SiLU, 2 LeakyReLU(0.2)");
+  SDW_REQUIRE(!d.resid2 || (d.resid && d.mode == GEMM_PLAIN), "a second residual needs a first one and plain mode");
   GemmKParams& p = L->p;
   std::memset(&p, 0, sizeof(p));
   const int kchunks = (d.C + BK - 1) / BK;
@@ -363,11 +366,12 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
   if (bn == 0) {
     if (d.mode == GEMM_GEGLU) bn = 128;
     else if (d.N % 160 == 0 && d.N % 128 != 0) bn = 160;
+    else if (d.N <= 32) bn = 32;
     else if (d.N <= 64) bn = 64;
     else bn = 128;
   }
-  SDW_REQUIRE(bn == 64 || bn == 128 || bn == 160 || bn == 256 || (bn == 192 && ver == 2), "unsupported BLOCK_N");
-  if (ver == 2) SDW_REQUIRE(bn != 64, "the 2-CTA kernel needs BLOCK_N >= 128");
+  SDW_REQUIRE(bn == 32 || bn == 64 || bn == 128 || bn == 160 || bn == 256 || (bn == 192 && ver == 2), "unsupported BLOCK_N");
+  if (ver == 2) SDW_REQUIRE(bn >= 128, "the 2-CTA kernel needs BLOCK_N >= 128");
   L->ver = ver;
   L->nsub = nsub;
   if (d.mode == GEMM_GEGLU) SDW_REQUIRE(bn % 64 == 0 && d.N % 64 == 0, "GEGLU needs 64-column pairs");
@@ -458,7 +462,7 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
     const bool vt_ok = d.mode != GEMM_QKV_VT ||
                        (Hd == 1 && bw == BM && d.conv == 0 && d.vt_col0 % 32 == 0 && d.vt_ld % 8 == 0 && ok16(d.vt) &&
                         d.vt_ntok == Wd && !d.resid);
-    bool can = nsub == 1 && !d.b_batched && vt_ok && (!d.rowvec || d.rowvec_ld == 0) &&
+    bool can = nsub == 1 && !d.b_batched && vt_ok && !d.resid2 && (!d.rowvec || d.rowvec_ld == 0) &&
                d.N % 8 == 0 && bn <= 256 && ok16(d.out) && ok_strides(osW, osH, osB) && (!d.bias || ok16(d.bias)) &&
                (!d.resid || (ok16(d.resid) && ok_strides(rsW, rsH, rsB) && d.mode == GEMM_PLAIN));
     if (d.et == 2) SDW_REQUIRE(can, "the TMA epilogue needs the CTA-pair kernel, plain/GEGLU mode, no row vector and 16-byte aligned views");
@@ -523,6 +527,8 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
   p.rowvec = d.rowvec;
   p.rowvec_ld = d.rowvec_ld;
   p.resid = d.resid;
+  p.resid2 = d.resid2;
+  p.res2_scale = d.res2_scale;
   p.out = d.out;
   if (d.o_sW || d.o_sH || d.o_sB) {
     p.o_sW = d.o_sW; p.o_sH = d.o_sH; p.o_sB = d.o_sB;
@@ -550,6 +556,9 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
 int launch_gemm(const GemmLaunch& l, cudaStream_t stream) {
   if (l.ver == 2) return launch_gemm2(l, stream);
   switch (l.bn) {
+    case 32:
+      SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<32>, l.grid, dim3(GEMM_THREADS), GemmCfg<32>::SMEM_BYTES, stream, l.p));
+      break;
     case 64:
       SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<64>, l.grid, dim3(GEMM_THREADS), GemmCfg<64>::SMEM_BYTES, stream, l.p));
       break;

@@ -1,6 +1,6 @@
 // sdw_gemm_epi.cuh — the fused epilogue shared by the 1-CTA and 2-CTA tcgen05 implicit-GEMM kernels:
-// TMEM accumulator (thread = output row) -> alpha / bias / time-embedding row / SiLU / residual / GEGLU /
-// per-head V^T scatter -> fp16 global stores.
+// TMEM accumulator (thread = output row) -> alpha / bias / time-embedding row / SiLU or LeakyReLU / residual /
+// scaled second residual / GEGLU / per-head V^T scatter -> fp16 global stores.
 #pragma once
 #include "sdw_internal.h"
 #include "sdw_ptx.cuh"
@@ -42,8 +42,10 @@ __device__ __forceinline__ void load8(const __half* src, float* v, bool vec_ok, 
 // fast paths: everything column-uniform is hoisted, 16-byte vector I/O only (the first version of this
 // epilogue spent ~750 SASS instructions per 32-column chunk on generic address / predicate math and was
 // the bottleneck of every short-K GEMM — see profiles/r01_ncu_gemm_linear_v1.txt).
-// FLAGS: 1 bias, 2 per-sample row vector (time embedding), 4 residual, 8 SiLU, 16 alpha != 1
+// FLAGS: 1 bias, 2 per-sample row vector (time embedding), 4 residual, 8 SiLU, 16 alpha != 1, 32 LeakyReLU(0.2)
 // ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ float leaky02(float x) { return x > 0.f ? x : 0.2f * x; }
+
 __device__ __forceinline__ void add8(float* o, const float* __restrict__ src) {
   const float4 a = __ldg(reinterpret_cast<const float4*>(src));
   const float4 b = __ldg(reinterpret_cast<const float4*>(src) + 1);
@@ -175,6 +177,10 @@ __device__ __forceinline__ void epi_fast(const GemmKParams& p, uint32_t taddr, i
 #pragma unroll
               for (int j = 0; j < 8; ++j) o[j] = silu_f(o[j]);
             }
+            if (FLAGS & 32) {
+#pragma unroll
+              for (int j = 0; j < 8; ++j) o[j] = leaky02(o[j]);
+            }
             if (FLAGS & 4) {
               const __half2* h = reinterpret_cast<const __half2*>(&rs[j8]);
 #pragma unroll
@@ -283,8 +289,11 @@ __device__ __forceinline__ void gemm_epilogue(const GemmKParams& p, uint32_t tme
   const float* rowvec = p.rowvec ? p.rowvec + static_cast<int64_t>(b) * p.rowvec_ld : nullptr;
   __half* out_row = p.out + out_off;
   const __half* res_row = p.resid ? p.resid + res_off : nullptr;
+  const __half* res2_row = p.resid2 ? p.resid2 + res_off : nullptr;
+  const bool vec_res2 = p.resid2 && (((p.r_sW | p.r_sH | p.r_sB) & 7) == 0) &&
+                        ((reinterpret_cast<uintptr_t>(p.resid2) & 15) == 0);
 
-  const bool fast = vec_out && (!p.resid || vec_res) && ((p.N & 7) == 0) &&
+  const bool fast = vec_out && (!p.resid || vec_res) && !p.resid2 && ((p.N & 7) == 0) &&
                     (!p.bias || (reinterpret_cast<uintptr_t>(p.bias) & 15) == 0) &&
                     (!p.rowvec || ((reinterpret_cast<uintptr_t>(p.rowvec) & 15) == 0 && (p.rowvec_ld & 3) == 0));
   // the residual does not depend on the accumulator: while the mainloop of this tile is still running, pull this
@@ -307,13 +316,16 @@ __device__ __forceinline__ void gemm_epilogue(const GemmKParams& p, uint32_t tme
   }
   if (fast) {
     const int flags = (p.bias ? 1 : 0) | (p.rowvec ? 2 : 0) | (p.resid ? 4 : 0) | (p.act == 1 ? 8 : 0) |
-                      (p.alpha != 1.f ? 16 : 0);
+                      (p.alpha != 1.f ? 16 : 0) | (p.act == 2 ? 32 : 0);
     switch (flags) {
       case 0: epi_fast<BN, 0>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
       case 1: epi_fast<BN, 1>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
       case 3: epi_fast<BN, 3>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
       case 5: epi_fast<BN, 5>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
       case 16: epi_fast<BN, 16>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
+      // Real-ESRGAN: conv + LeakyReLU, and the dense-block exit 0.2 * (acc + b) + x (bias pre-scaled)
+      case 33: epi_fast<BN, 33>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
+      case 21: epi_fast<BN, 21>(p, taddr, n0, row_ok, pix_in, out_row, res_row, rowvec, chunk0, chunk_step, stage, lane, out_off, g); return;
       default: break;
     }
   }
@@ -344,6 +356,7 @@ __device__ __forceinline__ void gemm_epilogue(const GemmKParams& p, uint32_t tme
           if (rowvec) a += __ldg(&rowvec[nn + j]);
         }
         if (p.act == 1) a = silu_f(a);
+        else if (p.act == 2) a = leaky02(a);
         o[j] = a;
       }
       if (p.resid) {
@@ -351,6 +364,12 @@ __device__ __forceinline__ void gemm_epilogue(const GemmKParams& p, uint32_t tme
         load8(res_row + nn, rr, vec_res, nvalid);
 #pragma unroll
         for (int j = 0; j < 8; ++j) o[j] += rr[j];
+      }
+      if (res2_row) {
+        float rr[8];
+        load8(res2_row + nn, rr, vec_res2, nvalid);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) o[j] = fmaf(o[j], p.res2_scale, rr[j]);
       }
       store8(out_row + nn, o, vec_out, nvalid);
     }
@@ -456,7 +475,7 @@ __device__ __forceinline__ void gemm_epilogue_tma(const GemmKParams& p, uint32_t
   }
 
   const int nch = (nmax + 31) >> 5;
-  const bool silu = p.act == 1;
+  const int act = p.act;
   const bool vt_mode = p.mode == GEMM_QKV_VT;
 #pragma unroll 1
   for (int c = cpar; c < nch; c += EW) {
@@ -515,9 +534,14 @@ __device__ __forceinline__ void gemm_epilogue_tma(const GemmKParams& p, uint32_t
           upk2(fma2(pk2(__uint_as_float(v[q * 8 + 2 * j]), __uint_as_float(v[q * 8 + 2 * j + 1])), alpha2, pk2(bv.x, bv.y)),
                o[2 * j], o[2 * j + 1]);
         }
-        if (silu) {
+        if (act) {  // one branch on the common act = 0 path
+          if (act == 1) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) o[j] = silu_f(o[j]);
+            for (int j = 0; j < 8; ++j) o[j] = silu_f(o[j]);
+          } else {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) o[j] = leaky02(o[j]);
+          }
         }
         if (rs) {
           const uint4 r4 = *reinterpret_cast<const uint4*>(rs + ((j8 ^ sw) << 4));

@@ -99,12 +99,15 @@ struct alignas(64) GemmKParams {
   int64_t o_sW, o_sH, o_sB;
   int os, ox, oy;
   int mode;
-  int act;                  // 0 none, 1 SiLU
+  int act;                  // 0 none, 1 SiLU, 2 LeakyReLU(0.2)
   float alpha;              // scale on the accumulator (before bias)
   // GEMM_QKV_VT
   int vt_col0, vt_d, vt_heads, vt_ntok;
   __half* vt;               // [b][head][d][vt_ld]
   int64_t vt_ld;
+  // second residual (generic epilogue only): out = res2_scale * (epilogue result incl. resid) + resid2, same strides as resid
+  const __half* resid2;
+  float res2_scale;
 };
 
 struct GemmLaunch {
@@ -141,8 +144,10 @@ struct GemmDesc {
   int64_t ldc = 0;                 // output pixel pitch; NHWC-contiguous output unless o_s* are given
   int64_t o_sW = 0, o_sH = 0, o_sB = 0;
   int mode = GEMM_PLAIN;
-  int act = 0;
+  int act = 0;                     // 0 none, 1 SiLU, 2 LeakyReLU(0.2)
   float alpha = 1.f;
+  const __half* resid2 = nullptr;  // second residual on the residual's strides: out = res2_scale * out + resid2
+  float res2_scale = 1.f;
   int vt_col0 = 0, vt_d = 0, vt_heads = 0, vt_ntok = 0;
   __half* vt = nullptr;
   int64_t vt_ld = 0;
@@ -225,8 +230,12 @@ int layernorm(const __half* x, int64_t ldx, int64_t rows, int C, const float* ga
 int softmax_rows(__half* s, int64_t ld, int64_t rows, int n, cudaStream_t stream);
 int conv_in_small(const __half* x, int64_t ldx, int B, int H, int W, int Cin, const __half* w, const float* bias,
                   int N, __half* y, int64_t ldy, cudaStream_t stream);
+// 3x3 conv of a uint8 RGB NHWC image read as x / 255 (Real-ESRGAN conv_first), OIHW fp16 weights [N][3][3][3]
+int conv_in_u8(const uint8_t* x, int B, int H, int W, const __half* w, const float* bias, int N, __half* y,
+               int64_t ldy, cudaStream_t stream);
+// unit01 = 0: uint8 = round(clamp(v/2+0.5, 0, 1)*255) (VAE); 1: round(clamp(v, 0, 1)*255) (Real-ESRGAN)
 int conv_out_small(const __half* x, int64_t ldx, int B, int H, int W, int C, const __half* w, const float* bias,
-                   int nout, float* out_f32, uint8_t* out_u8, cudaStream_t stream);
+                   int nout, float* out_f32, uint8_t* out_u8, cudaStream_t stream, int unit01 = 0);
 int vae_in(const float* x, float inv_scale, const __half* w, const float* bias, int F, int C, int H, int W, __half* z,
            cudaStream_t stream);
 int linear_f32(const float* in, int64_t ldi, const __half* w, const float* bias, int M, int N, int K, int silu_in,

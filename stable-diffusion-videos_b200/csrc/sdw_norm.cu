@@ -557,38 +557,44 @@ int softmax_rows(__half* s, int64_t ld, int64_t rows, int n, cudaStream_t stream
 // registers), loops over a tile of pixels whose 3x3xCin patches sit in shared memory.
 // w layout: [N][Cin][3][3] fp16 (the checkpoint's OIHW), bias fp32.
 // =============================================================================================
-template <int CIN>
-__global__ void __launch_bounds__(512) conv_in_kernel(const __half* __restrict__ x, int64_t ldx, int B, int H, int W,
+__device__ __forceinline__ float in_val(__half v) { return __half2float(v); }
+__device__ __forceinline__ float in_val(uint8_t v) { return static_cast<float>(v) / 255.f; }  // Real-ESRGAN: img / 255
+
+template <int CIN, typename TIn = __half>
+__global__ void __launch_bounds__(512) conv_in_kernel(const TIn* __restrict__ x, int64_t ldx, int B, int H, int W,
                                                        const __half* __restrict__ w, const float* __restrict__ bias,
                                                        int N, __half* __restrict__ y, int64_t ldy,
                                                        int pix_per_block) {
   // patch[pair][k] = (x of pixel 2*pair, x of pixel 2*pair + 1) for the 9*CIN taps: one 16-byte broadcast read feeds two
   // packed FMAs (two taps x two pixels); thread = output channel, its 9*CIN weights live in registers
   constexpr int K = 9 * CIN;
-  extern __shared__ float2 patch2[];  // [pix_per_block / 2][K]
+  constexpr int KP = (K + 1) & ~1;  // an even row length keeps the 16-byte reads aligned; the pad tap is zero
+  extern __shared__ float2 patch2[];  // [pix_per_block / 2][KP]
   const int64_t P = static_cast<int64_t>(B) * H * W;
   const int64_t p0 = static_cast<int64_t>(blockIdx.x) * pix_per_block;
   const int np = static_cast<int>(min(static_cast<int64_t>(pix_per_block), P - p0));
   pdl_wait();
   pdl_launch_dependents();
-  for (int i = threadIdx.x; i < pix_per_block * K; i += blockDim.x) {
-    const int c = i % CIN;
-    const int tap = (i / CIN) % 9;
-    const int lp = i / K;
+  for (int i = threadIdx.x; i < pix_per_block * KP; i += blockDim.x) {
+    const int k = i % KP;
+    const int c = k % CIN;
+    const int tap = k / CIN;
+    const int lp = i / KP;
     const int64_t p = p0 + lp;
     float v = 0.f;
-    if (lp < np) {
+    if (lp < np && k < K) {
       const int xw = static_cast<int>(p % W), yh = static_cast<int>((p / W) % H);
       const int64_t b = p / (static_cast<int64_t>(W) * H);
       const int yy = yh + tap / 3 - 1, xx = xw + tap % 3 - 1;
-      if (yy >= 0 && yy < H && xx >= 0 && xx < W) v = __half2float(x[((b * H + yy) * W + xx) * ldx + c]);
+      if (yy >= 0 && yy < H && xx >= 0 && xx < W) v = in_val(x[((b * H + yy) * W + xx) * ldx + c]);
     }
-    reinterpret_cast<float*>(patch2)[((lp >> 1) * K + tap * CIN + c) * 2 + (lp & 1)] = v;
+    reinterpret_cast<float*>(patch2)[((lp >> 1) * KP + k) * 2 + (lp & 1)] = v;
   }
   __syncthreads();
   const int n = threadIdx.x;
   if (n >= N) return;
-  uint64_t wr[K];
+  uint64_t wr[KP];
+  wr[KP - 1] = 0;
 #pragma unroll
   for (int tap = 0; tap < 9; ++tap)
 #pragma unroll
@@ -599,9 +605,9 @@ __global__ void __launch_bounds__(512) conv_in_kernel(const __half* __restrict__
   const float bn = bias ? bias[n] : 0.f;
   for (int pr = 0; pr * 2 < np; ++pr) {
     uint64_t acc = pk2(bn, bn);
-    const float4* row = reinterpret_cast<const float4*>(patch2 + pr * K);
+    const float4* row = reinterpret_cast<const float4*>(patch2 + pr * KP);
 #pragma unroll
-    for (int k = 0; k < K / 2; ++k) {
+    for (int k = 0; k < KP / 2; ++k) {
       const float4 v = row[k];
       acc = fma2(pk2(v.x, v.y), wr[2 * k], acc);
       acc = fma2(pk2(v.z, v.w), wr[2 * k + 1], acc);
@@ -626,16 +632,29 @@ int conv_in_small(const __half* x, int64_t ldx, int B, int H, int W, int Cin, co
   return 0;
 }
 
+int conv_in_u8(const uint8_t* x, int B, int H, int W, const __half* w, const float* bias, int N, __half* y,
+               int64_t ldy, cudaStream_t stream) {
+  SDW_REQUIRE(N <= 512, "conv_in: N <= 512");
+  const int ppb = 64;
+  const int64_t P = static_cast<int64_t>(B) * H * W;
+  const int threads = (N + 31) / 32 * 32;
+  conv_in_kernel<3, uint8_t><<<static_cast<unsigned>((P + ppb - 1) / ppb), threads, ppb * 28 * sizeof(float), stream>>>(
+      x, 3, B, H, W, w, bias, N, y, ldy, ppb);
+  SDW_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
 // =============================================================================================
 // conv_out: 3x3 pad 1, C -> NOUT (<= 4) channels, one warp per output pixel; lanes split the channels.
 // Input is the already normalised + SiLU'd fp16 NHWC tensor.  w layout: OIHW fp16 [NOUT][C][3][3].
 //   out_f32  : fp32 NHWC [P][NOUT] (UNet eps)          — optional
-//   out_u8   : uint8 NHWC [P][NOUT] = round(clamp(v/2+0.5,0,1)*255) (VAE frame; P:435-438 + numpy_to_pil) — optional
+//   out_u8   : uint8 NHWC [P][NOUT] = round(clamp(v/2+0.5,0,1)*255) (VAE frame; P:435-438 + numpy_to_pil) — optional;
+//              UNIT01: round(clamp(v,0,1)*255) (Real-ESRGAN's output post-process)
 // =============================================================================================
 // A block owns a TS x TS pixel tile: its (TS+2)^2 halo is staged once in shared memory (the row-per-warp version
 // re-read every input pixel nine times from L2: 245 us for the UNet's 320->4 conv, ~6 ms for the VAE's 128->3), the
 // weights sit next to it; a warp computes 8 pixels at a time, lanes split the channels, one tap's weights in registers.
-template <int NOUT, int TS>
+template <int NOUT, int TS, bool UNIT01 = false>
 __global__ void __launch_bounds__(256) conv_out_kernel(const __half* __restrict__ x, int64_t ldx, int B, int H, int W,
                                                        int C, const __half* __restrict__ w,
                                                        const float* __restrict__ bias, float* __restrict__ out_f32,
@@ -749,7 +768,7 @@ __global__ void __launch_bounds__(256) conv_out_kernel(const __half* __restrict_
             const float v = acc[j][n] + (bias ? bias[n] : 0.f);
             if (out_f32) out_f32[p * NOUT + n] = v;
             if (out_u8) {
-              const float q = fminf(fmaxf(v * 0.5f + 0.5f, 0.f), 1.f);
+              const float q = fminf(fmaxf(UNIT01 ? v : v * 0.5f + 0.5f, 0.f), 1.f);
               out_u8[p * NOUT + n] = static_cast<uint8_t>(rintf(q * 255.f));
             }
           }
@@ -760,29 +779,34 @@ __global__ void __launch_bounds__(256) conv_out_kernel(const __half* __restrict_
   }  // tile loop
 }
 
-template <int NOUT, int TS>
+template <int NOUT, int TS, bool UNIT01 = false>
 static int launch_conv_out(const __half* x, int64_t ldx, int B, int H, int W, int C, const __half* w, const float* bias,
                            float* out_f32, uint8_t* out_u8, cudaStream_t stream) {
   const size_t smem = (static_cast<size_t>((TS + 2) * (TS + 2)) + NOUT * 9) * C * sizeof(__half);
   SDW_REQUIRE(smem <= 227 * 1024, "conv_out: channel count too large for the halo tile");
   static bool attr_done = false;
   if (!attr_done) {
-    SDW_CUDA_OK(cudaFuncSetAttribute(conv_out_kernel<NOUT, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    SDW_CUDA_OK(cudaFuncSetAttribute(conv_out_kernel<NOUT, TS, UNIT01>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     attr_done = true;
   }
   const int64_t tiles = static_cast<int64_t>(B) * ((H + TS - 1) / TS) * ((W + TS - 1) / TS);
   const int64_t blocks = std::min<int64_t>(tiles, 148 * 2);  // persistent: the weights are staged once per block
-  conv_out_kernel<NOUT, TS><<<static_cast<unsigned>(blocks), 256, smem, stream>>>(x, ldx, B, H, W, C, w, bias, out_f32, out_u8);
+  conv_out_kernel<NOUT, TS, UNIT01><<<static_cast<unsigned>(blocks), 256, smem, stream>>>(x, ldx, B, H, W, C, w, bias, out_f32, out_u8);
   SDW_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
 int conv_out_small(const __half* x, int64_t ldx, int B, int H, int W, int C, const __half* w, const float* bias,
-                   int nout, float* out_f32, uint8_t* out_u8, cudaStream_t stream) {
+                   int nout, float* out_f32, uint8_t* out_u8, cudaStream_t stream, int unit01) {
   SDW_REQUIRE(nout == 3 || nout == 4, "conv_out: 3 or 4 output channels");
   SDW_REQUIRE(C % 8 == 0 && ldx % 8 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0, "conv_out: 16-byte aligned channel rows");
   // 16 x 16 tiles when their halo fits comfortably (C <= 128), 8 x 8 otherwise
   const bool big = C <= 128 && H >= 16 && W >= 16;
+  if (unit01) {
+    SDW_REQUIRE(nout == 3, "conv_out: the [0, 1] post-process is for RGB output");
+    return big ? launch_conv_out<3, 16, true>(x, ldx, B, H, W, C, w, bias, out_f32, out_u8, stream)
+               : launch_conv_out<3, 8, true>(x, ldx, B, H, W, C, w, bias, out_f32, out_u8, stream);
+  }
   if (nout == 4)
     return big ? launch_conv_out<4, 16>(x, ldx, B, H, W, C, w, bias, out_f32, out_u8, stream)
                : launch_conv_out<4, 8>(x, ldx, B, H, W, C, w, bias, out_f32, out_u8, stream);

@@ -451,7 +451,13 @@ class StableDiffusionWalkPipeline:
         if T.shape[0] != num_interpolation_steps:
             raise ValueError(f"Unexpected T shape, got {T.shape}, expected dim 0 to be {num_interpolation_steps}")
         if upsample:
-            raise NotImplementedError("Real-ESRGAN upsampling is outside the hot path (SURVEY.md §2 #5)")
+            if self.upsampler is None:
+                raise ValueError("upsample=True needs a Real-ESRGAN upsampler: set "
+                                 "`pipe.upsampler = RealESRGANModel.from_pretrained(local_path)` (a local "
+                                 "RealESRGAN_x4plus.pth; nothing is downloaded)")
+            if self.tiled:
+                raise NotImplementedError("upsample=True with tiled=True (a circularly padded upsampler) is not "
+                                          "implemented")
         if height % 8 != 0 or width % 8 != 0:  # raised by __call__ in the reference (P:271-272)
             raise ValueError(f"`height` and `width` have to be divisible by 8 but are {height} and {width}.")
         if eta != 0.0 and type(self.scheduler).__name__.startswith("DDIM"):
@@ -466,6 +472,9 @@ class StableDiffusionWalkPipeline:
         uncond = self._uncond([negative_prompt if negative_prompt is not None else ""]) if do_cfg else None
         # decoded frame size = latent size x vae_scale_factor (the reference hard-codes // 8 for the latents, P:368)
         out_h, out_w = h8 * self.vae_scale_factor, w8 * self.vae_scale_factor
+        if upsample:  # every rank upsamples its own frames on its device, before the gather and the sink
+            self.upsampler.to(self.device)
+            out_h, out_w = 4 * out_h, 4 * out_w
         sink = _FrameSink(save_path, image_file_ext, (batch_size, out_h, out_w, self.vae.cfg.out_channels),
                           self.device) if rank == 0 else None
         mine = []  # this rank's frames, on the device, when they have to travel to rank 0
@@ -480,6 +489,8 @@ class StableDiffusionWalkPipeline:
                 noise_batch = torch.cat([noise_batch, noise_batch[-1:].expand(pad, -1, -1, -1)])
             frames_u8, _ = self._sample_device(noise_batch, embeds_batch, uncond, height, width, num_inference_steps,
                                                guidance_scale)
+            if upsample:
+                frames_u8 = self.upsampler.upsample_frames(frames_u8[:nb])
             if world > 1:
                 mine.append(frames_u8[:nb].clone())
             else:
