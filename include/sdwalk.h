@@ -189,9 +189,11 @@ typedef struct sdw_gemm_desc {
   int32_t vt_col0, vt_d, vt_heads, vt_ntok;
   void* vt;
   int64_t vt_ld;
-  int32_t bn;                /* BLOCK_N: 0 auto, 32/64/128/160/256 (32 and 64: one-CTA kernel only) */
+  int32_t bn;                /* BLOCK_N: 0 auto, 32/64/128/160/192/256 (32 and 64: one-CTA kernel only; 192 and 256:
+                              * CTA-pair kernel only) */
   int32_t ver;               /* 0 auto, 1: one CTA per 128xBN tile, 2: persistent CTA pairs (256xBN) */
-  int32_t nsub;              /* 0 auto, 1 / 2: accumulators per activation tile in the CTA-pair kernel */
+  int32_t nsub;              /* 0 auto, 1 / 2: accumulators per activation tile in the CTA-pair kernel (2: not with tap
+                              * reuse; it turns the automatic tap reuse off) */
   int32_t ew;                /* 0 auto, 2 / 4: epilogue warps per TMEM lane quarter of the CTA-pair kernel (4: needs the TMA epilogue) */
   int32_t tr;                /* 0 auto, 1 never, 2 require: 3x3 taps reuse one activation box in shared memory */
   int32_t et;                /* 0 auto, 1 never, 2 require: TMA-store epilogue with a TMA-fed residual ring.  With mode 2 the

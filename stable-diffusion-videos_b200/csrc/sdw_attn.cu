@@ -32,7 +32,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 namespace sdw {
@@ -110,7 +109,7 @@ struct PPCfg {
 
 // TRACE: compile the clock64 stamps in (tools/attn_trace.py); the shipped instantiation carries no trace code — with the
 // stamps merely predicated off the kernel was 8 % slower
-template <int DVP, int TRACE, int POLY>
+template <int DVP, int TRACE>
 __global__ void __launch_bounds__(PPCfg<DVP>::THREADS, 1) attn_pp_kernel(const __grid_constant__ AttnKParams p) {
   using Cfg = PPCfg<DVP>;
   constexpr int ST = Cfg::ST, BKV = 128;
@@ -161,8 +160,6 @@ __global__ void __launch_bounds__(PPCfg<DVP>::THREADS, 1) attn_pp_kernel(const _
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_ptr_smem;
-  pdl_wait();
-  pdl_launch_dependents();
 
   if (warp < 4) {
     reg_dealloc<Cfg::REGS_OTHER>();
@@ -321,8 +318,8 @@ __global__ void __launch_bounds__(PPCfg<DVP>::THREADS, 1) attn_pp_kernel(const _
         }
         if (trace) ts3 = clock64();
         // ---- exponentials against the reference max, P -> tensor memory chunk by chunk.  One pair in four goes through
-        //      the FMA pipe (POLY = 4): same box, batch 60: 4.18 M cycles against 4.43 M with every exponential on the
-        //      MUFU (profiles/r02_attn_softmax_loop_ab_same_box.txt) -------------------------------------------------
+        //      the FMA pipe: same box, batch 60: 4.18 M cycles against 4.43 M with every exponential on the MUFU
+        //      (profiles/r02_attn_softmax_loop_ab_same_box.txt) ----------------------------------------------------------
         const float mb = m_ref * sl2;
         const uint64_t sl2_2 = pk2(sl2, sl2), nmb_2 = pk2(-mb, -mb);
         uint64_t sm2[4] = {pk2(0.f, 0.f), pk2(0.f, 0.f), pk2(0.f, 0.f), pk2(0.f, 0.f)};
@@ -340,7 +337,7 @@ __global__ void __launch_bounds__(PPCfg<DVP>::THREADS, 1) attn_pp_kernel(const _
             upk2(fma2(pk2(__uint_as_float(v[c][i + 2]), __uint_as_float(v[c][i + 3])), sl2_2, nmb_2), t2, t3);
             e0 = ex2f(t0);
             e1 = ex2f(t1);
-            if (POLY && ((i >> 2) % POLY) == POLY - 1) {
+            if ((i >> 2) % 4 == 3) {
               ex2_poly2(t2, t3, e2, e3);  // this pair on the FMA pipe
             } else {
               e2 = ex2f(t2);
@@ -494,8 +491,6 @@ __global__ void __launch_bounds__(ATT_THREADS, AttnCfg<DKA, DVP, BKV, ST, SB, PT
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_ptr_smem;
-  pdl_wait();
-  pdl_launch_dependents();
 
   if (warp == 0) {
     // ============================ TMA producer ============================================
@@ -813,16 +808,17 @@ static int attn_set_attr() {
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, AttnCfg<DKA, DVP, BKV, ST, SB, PT>::SMEM));
   return 0;
 }
-template <int DVP, int TRACE, int POLY>
+template <int DVP, int TRACE>
 static cudaError_t pp_launch_one(const AttnKParams& p, dim3 grid, cudaStream_t stream) {
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(attn_pp_kernel<DVP, TRACE, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(attn_pp_kernel<DVP, TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          PPCfg<DVP>::SMEM);
     if (e != cudaSuccess) return e;
     attr = true;
   }
-  return launch_pdl(attn_pp_kernel<DVP, TRACE, POLY>, grid, dim3(PPCfg<DVP>::THREADS), PPCfg<DVP>::SMEM, stream, p);
+  attn_pp_kernel<DVP, TRACE><<<grid, PPCfg<DVP>::THREADS, PPCfg<DVP>::SMEM, stream>>>(p);
+  return cudaGetLastError();
 }
 
 static bool g_attn_init = false;
@@ -844,13 +840,10 @@ static long long* g_attn_dbg = nullptr;
 void attention_set_trace(long long* buf) { g_attn_dbg = buf; }
 
 static int variant_for(int d, int Nk, int Nq) {
-  // SDW_ATTN_PP=0: the one-query-tile kernel everywhere (A/B measurements)
-  static const bool pp = [] { const char* e = std::getenv("SDW_ATTN_PP"); return !(e && e[0] == '0'); }();
   const int cls = d <= 16 ? 0 : (d <= 32 ? 1 : (d <= 48 ? 2 : 3));
   // single-KV-tile (cross) attention with >= 2 query tiles goes through the two-tile kernel as well: 64x64, 77 keys,
-  // batch 60: 155.6 us against 193.1 us for the query-tile loop of attn_fwd_kernel (same box); SDW_ATTN_PP_CROSS=0 = A/B
-  static const bool pp_cross = [] { const char* e = std::getenv("SDW_ATTN_PP_CROSS"); return !(e && e[0] == '0'); }();
-  if (d <= 64) return (pp && (Nk > 128 || (pp_cross && Nq >= 256))) ? 8 + cls : cls;
+  // batch 60: 155.6 us against 193.1 us for the query-tile loop of attn_fwd_kernel (same box)
+  if (d <= 64) return (Nk > 128 || Nq >= 256) ? 8 + cls : cls;
   return d <= 80 ? 4 : 5;
 }
 
@@ -930,19 +923,15 @@ void attention_plan_info(const AttnLaunch& L, int out[5]) {
 
 template <int DKA, int DVP, int BKV, int ST, int SB, int PT>
 static cudaError_t launch_fwd(const AttnLaunchImpl* I, cudaStream_t stream) {
-  return launch_pdl(attn_fwd_kernel<DKA, DVP, BKV, ST, SB, PT>, I->grid, dim3(ATT_THREADS),
-                    AttnCfg<DKA, DVP, BKV, ST, SB, PT>::SMEM, stream, I->p);
+  attn_fwd_kernel<DKA, DVP, BKV, ST, SB, PT><<<I->grid, ATT_THREADS, AttnCfg<DKA, DVP, BKV, ST, SB, PT>::SMEM, stream>>>(I->p);
+  return cudaGetLastError();
 }
-static constexpr int PP_POLY = 4;  // shipped: one exponential pair in four on the FMA pipe
 template <int DVP>
 static cudaError_t launch_pp(const AttnLaunchImpl* I, cudaStream_t stream) {
   AttnKParams p = I->p;
   p.dbg = g_attn_dbg;
-  // SDW_ATTN_POLY=0: every exponential on the MUFU (the A/B leg of tools/attn_bench.py)
-  static const int poly = [] { const char* e = std::getenv("SDW_ATTN_POLY"); return e ? std::atoi(e) : PP_POLY; }();
-  if (p.dbg) return pp_launch_one<DVP, 1, PP_POLY>(p, I->grid, stream);
-  if (poly == 0) return pp_launch_one<DVP, 0, 0>(p, I->grid, stream);
-  return pp_launch_one<DVP, 0, PP_POLY>(p, I->grid, stream);
+  if (p.dbg) return pp_launch_one<DVP, 1>(p, I->grid, stream);
+  return pp_launch_one<DVP, 0>(p, I->grid, stream);
 }
 
 int launch_attention(const AttnLaunch& L, cudaStream_t stream) {

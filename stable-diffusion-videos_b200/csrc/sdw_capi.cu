@@ -2,16 +2,11 @@
 #include "../../include/sdwalk.h"
 #include "sdw_internal.h"
 
-#include <cstdlib>
 #include <cstring>
 
 namespace sdw {
 static thread_local std::string g_err;
 void set_error(const std::string& msg) { g_err = msg; }
-bool pdl_enabled() {
-  static const bool on = [] { const char* e = std::getenv("SDW_PDL"); return e && e[0] == '1'; }();  // measured no gain: opt-in
-  return on;
-}
 const char* last_error() { return g_err.c_str(); }
 }  // namespace sdw
 

@@ -15,7 +15,6 @@
 #include "sdw_internal.h"
 
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <functional>
 #include <map>
@@ -325,12 +324,11 @@ struct Engine {
     emit([=](cudaStream_t st, int) { return layernorm(x.p, x.ld, x.pixels(), x.C, g, b, 1e-5f, out.p, out.ld, st); });
   }
   int cfg_groups = 32;
-  bool use_flash = true;
 
   // unfused attention: S = alpha Q K^T (head-batched tcgen05 GEMM) ; softmax rows ; O = P V
   int attention(const __half* q, int64_t q_ld, const __half* k, int64_t k_ld, const __half* vt, int64_t vt_ld, int Bq,
                 int Nq, int Nk, int heads, int d, const T& out) {
-    if (use_flash && attn_supported(d)) {
+    if (attn_supported(d)) {
       if (dry) {
         *cur_count += 1;
         return 0;
@@ -766,13 +764,13 @@ struct Engine {
     out_img_f32 = static_cast<float*>(alloc(static_cast<size_t>(F) * OH * OW * cfg.vae_out_channels * 4));
     gn_ws = static_cast<float2*>(alloc(gn_workspace_bytes(std::max(Bn, F))));
     // attention score scratch of the UNFUSED path: the VAE mid attention (d = 512), and UNet level-0 self attention only
-    // when its head dim has no fused kernel (or SDW_NO_FLASH)
+    // when its head dim has no fused kernel
     {
       const int64_t n0 = static_cast<int64_t>(H) * W;
       int64_t unet_s = 0;
       for (int l = 0; l < cfg.num_levels; ++l) {
         const int hl = std::max(1, cfg.attention_heads[l]);
-        if (use_flash && attn_supported(cfg.block_out_channels[l] / hl)) continue;
+        if (attn_supported(cfg.block_out_channels[l] / hl)) continue;
         const int64_t nl = static_cast<int64_t>(H >> l) * (W >> l);
         const int64_t nlp = (nl + 7) / 8 * 8;
         unet_s = std::max(unet_s, static_cast<int64_t>(unfused_chunk(Bn, hl, nl, nlp)) * hl * nl * nlp);
@@ -856,7 +854,6 @@ int sdw_engine_create(const sdw_engine_config* cfg, sdw_engine** out) {
   Engine* E = new Engine();
   E->cfg = *cfg;
   E->tiled = cfg->tiled != 0;
-  if (const char* nf = std::getenv("SDW_NO_FLASH")) E->use_flash = !(nf[0] == '1');
   if (int e = E->build(true, nullptr)) {
     delete E;
     return e;

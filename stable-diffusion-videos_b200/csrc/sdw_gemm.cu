@@ -19,7 +19,6 @@
 #include <cudaTypedefs.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 
 namespace sdw {
@@ -32,7 +31,7 @@ static constexpr int GEMM_THREADS = 192;
 template <int BN>
 struct GemmCfg {
   static constexpr int B_STAGE_BYTES = BN * BK * 2;
-  static constexpr int STAGES = (BN <= 64) ? 4 : (BN <= 160 ? 3 : 4);
+  static constexpr int STAGES = BN <= 64 ? 4 : 3;
   static constexpr int TMEM_COLS = BN <= 32 ? 32 : (BN <= 64 ? 64 : (BN <= 128 ? 128 : 256));
   static constexpr int SMEM_BYTES = STAGES * (A_STAGE_BYTES + B_STAGE_BYTES) + 1024 /*align*/ + 256 /*barriers*/;
 };
@@ -81,8 +80,6 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_tc_kernel(const __grid_cons
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_acc = *tmem_ptr_smem;
-  pdl_wait();
-  pdl_launch_dependents();
 
   if (warp == 0) {
     // =========================== TMA producer ===============================
@@ -170,7 +167,6 @@ int gemm_init() {
   if (int e = set_attr<64>()) return e;
   if (int e = set_attr<128>()) return e;
   if (int e = set_attr<160>()) return e;
-  if (int e = set_attr<256>()) return e;
   return 0;
 }
 
@@ -303,18 +299,16 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
   // kernel version: CTA pairs need >= 2 M tiles and a wide-enough N; batched matmuls must pair within one (h, b)
   const int m_tiles = p.tiles_w * p.tiles_h * tiles_b;
   int ver = d.ver;
-  if (ver == 0) {
-    static const bool force_v1 = [] { const char* e = std::getenv("SDW_GEMM_V1"); return e && e[0] == '1'; }();
-    ver = (!force_v1 && m_tiles >= 2 && d.N >= 128 && (!d.b_batched || p.tiles_w % 2 == 0)) ? 2 : 1;
-  }
+  if (ver == 0) ver = (m_tiles >= 2 && d.N >= 128 && (!d.b_batched || p.tiles_w % 2 == 0)) ? 2 : 1;
   if (ver == 2) SDW_REQUIRE(!d.b_batched || p.tiles_w % 2 == 0, "2-CTA batched matmul needs an even tile count per row");
-  // tap reuse (3x3 stride 1, CTA pairs): 16 x 8-pixel tiles, one 10-row activation box per (channel chunk, kx)
+  // tap reuse (3x3 stride 1, CTA pairs): 16 x 8-pixel tiles, one 10-row activation box per (channel chunk, kx).  Only
+  // two operand stages of the two-accumulator tile would fit next to the 3-tap boxes, so two accumulators mean per-tap loads.
   bool reuse = false;
   {
-    static const int tr_env = [] { const char* e = std::getenv("SDW_GEMM_TR"); return e ? std::atoi(e) : -1; }();
     const bool can = ver == 2 && d.conv == 1 && Wd % 16 == 0 && Hd % 8 == 0;
     if (d.tr == 2) SDW_REQUIRE(can, "tap reuse needs a 3x3 stride-1 conv on the CTA-pair kernel with W % 16 == 0, H % 8 == 0");
-    reuse = can && d.tr != 1 && (d.tr == 2 || tr_env != 0);
+    if (d.tr == 2) SDW_REQUIRE(d.nsub != 2, "two accumulators per activation tile need the per-tap mainloop, not tap reuse");
+    reuse = can && d.tr != 1 && d.nsub != 2;
     if (reuse) {
       p.bw = bw = 16;
       p.bh = bh = 8;
@@ -346,7 +340,7 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
       if (d.bn && d.bn != c.bn) continue;
       if (d.nsub && d.nsub != c.nsub) continue;
       if (d.mode == GEMM_GEGLU && c.bn % 64 != 0) continue;
-      if (c.nsub == 2 && (kblocks < 18 || d.mode != GEMM_PLAIN || reuse) && d.nsub != 2) continue;  // reuse: only 2 stages fit
+      if (c.nsub == 2 && (kblocks < 18 || d.mode != GEMM_PLAIN || reuse) && d.nsub != 2) continue;
       const int width = c.bn * c.nsub;
       const int tiles = mp * ((d.N + width - 1) / width);
       const int waves = (tiles + 73) / 74;
@@ -370,7 +364,8 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
     else if (d.N <= 64) bn = 64;
     else bn = 128;
   }
-  SDW_REQUIRE(bn == 32 || bn == 64 || bn == 128 || bn == 160 || bn == 256 || (bn == 192 && ver == 2), "unsupported BLOCK_N");
+  SDW_REQUIRE(bn == 32 || bn == 64 || bn == 128 || bn == 160 || ((bn == 192 || bn == 256) && ver == 2),
+              "unsupported BLOCK_N (192 and 256 need the CTA-pair kernel)");
   if (ver == 2) SDW_REQUIRE(bn >= 128, "the 2-CTA kernel needs BLOCK_N >= 128");
   L->ver = ver;
   L->nsub = nsub;
@@ -380,9 +375,8 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
   L->grid = dim3(m_tiles_f, (d.N + bn - 1) / bn, 1);
   {
     // store staging pays off when the epilogue, not the mainloop, bounds the tile (short K, wide N)
-    static const int stage_env = [] { const char* e = std::getenv("SDW_STAGE"); return e ? std::atoi(e) : -1; }();
     const int kblocks = p.ntaps * kchunks;
-    p.stage_stores = stage_env >= 0 ? stage_env : (kblocks <= 10 && d.N >= 640 ? 1 : 0);
+    p.stage_stores = kblocks <= 10 && d.N >= 640 ? 1 : 0;
     // the coalescing stage keeps 32-bit row offsets
     const int64_t max_off = static_cast<int64_t>(d.B) * OH * OW * std::max<int64_t>(d.ldc, d.ldr ? d.ldr : d.ldc);
     SDW_REQUIRE(max_off < (int64_t(1) << 31) || ver == 1, "output too large for the 2-CTA epilogue (>= 2^31 elements)");
@@ -466,13 +460,11 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
                d.N % 8 == 0 && bn <= 256 && ok16(d.out) && ok_strides(osW, osH, osB) && (!d.bias || ok16(d.bias)) &&
                (!d.resid || (ok16(d.resid) && ok_strides(rsW, rsH, rsB) && d.mode == GEMM_PLAIN));
     if (d.et == 2) SDW_REQUIRE(can, "the TMA epilogue needs the CTA-pair kernel, plain/GEGLU mode, no row vector and 16-byte aligned views");
-    static const int et_env = [] { const char* e = std::getenv("SDW_EPI_TMA"); return e ? std::atoi(e) : -1; }();
     const int kblocks = p.ntaps * kchunks;
     // short-K GEMMs are bound by their epilogue (profiles/r01_ncu_epilogue_shortk.md) and gain up to 2x; long-K ones
     // lose one operand stage to the epilogue buffers but still come out ahead end to end (bench: 8.49 -> 8.56 frames/s),
-    // so the TMA epilogue is used wherever it is eligible.  SDW_EPI_TMA=0 disables it, =2 restricts it to <= 24 K blocks.
-    const bool want = d.et == 2 || (d.et == 0 && (et_env < 0 || et_env == 1 || (et_env == 2 && kblocks <= 24)));
-    p.epi_tma = can && want ? 1 : 0;
+    // so the TMA epilogue is used wherever it is eligible
+    p.epi_tma = can && (d.et == 0 || d.et == 2) ? 1 : 0;
     const int a_stage = reuse ? 20480 : 16384;
     const int b_stage = (reuse ? 3 : 1) * nsub * (bn / 2) * 128;
     const int epi_bytes = p.epi_tma ? G2_EPI_OUT + G2_EPI_BIAS + (d.resid ? G2_RES_STAGES * G2_RES_STAGE : 0) : G2_EPI_OLD;
@@ -481,12 +473,11 @@ int plan_gemm(const GemmDesc& d, GemmLaunch* L) {
     // epilogue width: four warps per TMEM lane quarter where the epilogue, not the MMA, sets the tile time — K <= 448
     // (the 64x64-level transformer linears, K = 320: GEGLU 434 -> 383 us, QKV-like 218 -> 161 us, out-projection 99 ->
     // 88 us at batch 60, same box; from K = 640 on the MMA is the longer leg and the wider epilogue loses 2-10 %:
-    // profiles/r02_epilogue_width_ab_same_box.txt).  SDW_GEMM_EW=2 | 4: 8-warp epilogue everywhere / 16 wherever eligible
+    // profiles/r02_epilogue_width_ab_same_box.txt)
     {
-      static const int ew_env = [] { const char* e = std::getenv("SDW_GEMM_EW"); return e ? std::atoi(e) : 0; }();
       const bool can4 = p.epi_tma && nsub == 1 && !reuse;
       if (d.ew == 4) SDW_REQUIRE(can4, "the 16-warp epilogue needs the TMA epilogue, one accumulator and the per-tap mainloop");
-      const int want4 = d.ew ? d.ew == 4 : (ew_env ? ew_env == 4 : kblocks <= 7);
+      const int want4 = d.ew ? d.ew == 4 : kblocks <= 7;
       L->ew = can4 && want4 ? 4 : 2;
       if (L->ew == 4) {  // 16 per-warp bias copies instead of 8, eight residual ring slots instead of four
         const int extra = G2_EPI_BIAS + (d.resid ? G2_RES_STAGES * G2_RES_STAGE : 0);
@@ -557,19 +548,16 @@ int launch_gemm(const GemmLaunch& l, cudaStream_t stream) {
   if (l.ver == 2) return launch_gemm2(l, stream);
   switch (l.bn) {
     case 32:
-      SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<32>, l.grid, dim3(GEMM_THREADS), GemmCfg<32>::SMEM_BYTES, stream, l.p));
+      gemm_tc_kernel<32><<<l.grid, GEMM_THREADS, GemmCfg<32>::SMEM_BYTES, stream>>>(l.p);
       break;
     case 64:
-      SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<64>, l.grid, dim3(GEMM_THREADS), GemmCfg<64>::SMEM_BYTES, stream, l.p));
+      gemm_tc_kernel<64><<<l.grid, GEMM_THREADS, GemmCfg<64>::SMEM_BYTES, stream>>>(l.p);
       break;
     case 128:
-      SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<128>, l.grid, dim3(GEMM_THREADS), GemmCfg<128>::SMEM_BYTES, stream, l.p));
+      gemm_tc_kernel<128><<<l.grid, GEMM_THREADS, GemmCfg<128>::SMEM_BYTES, stream>>>(l.p);
       break;
     case 160:
-      SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<160>, l.grid, dim3(GEMM_THREADS), GemmCfg<160>::SMEM_BYTES, stream, l.p));
-      break;
-    case 256:
-      SDW_CUDA_OK(launch_pdl(gemm_tc_kernel<256>, l.grid, dim3(GEMM_THREADS), GemmCfg<256>::SMEM_BYTES, stream, l.p));
+      gemm_tc_kernel<160><<<l.grid, GEMM_THREADS, GemmCfg<160>::SMEM_BYTES, stream>>>(l.p);
       break;
     default:
       set_error("bad BLOCK_N");

@@ -137,8 +137,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G2Threads<EW>::value
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();               // the set-up above overlapped the previous kernel's tail; its outputs are visible from here
-  pdl_launch_dependents();  // let the next kernel's CTAs start their own set-up as soon as SMs free up
   auto tile_coords = [&](int t, int& x0, int& y0, int& b0, int& n0) {
     // N fastest: the n_tiles column tiles of one M pair run on neighbouring clusters at the same time, so the
     // activation tile is fetched from DRAM once and re-read from L2 (the whole weight matrix is L2-resident anyway)
@@ -330,16 +328,13 @@ static int launch2(const GemmLaunch& l, cudaStream_t stream) {
                                      Gemm2Cfg<BN, NSUB, TR>::SMEM_BYTES));
     attr = true;
   }
-  SDW_CUDA_OK(launch_pdl(gemm2_tc_kernel<BN, NSUB, EW, TR>, l.grid, dim3(G2Threads<EW>::value),
-                         Gemm2Cfg<BN, NSUB, TR>::SMEM_BYTES, stream, l.p));
+  gemm2_tc_kernel<BN, NSUB, EW, TR><<<l.grid, G2Threads<EW>::value, Gemm2Cfg<BN, NSUB, TR>::SMEM_BYTES, stream>>>(l.p);
   SDW_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-int gemm2_init() { return 0; }
-
-// instantiations: BLOCK_N 128 / 160 / 192 / 256 x {per-tap, tap reuse} with one accumulator, 160 x 2 accumulators; the
-// wide epilogue (EW = 4) for the per-tap kernels with one accumulator (the short-K linears / 1x1 convs)
+// instantiations: BLOCK_N 128 / 160 / 192 / 256 x {per-tap, tap reuse} with one accumulator, 160 x 2 accumulators
+// (per-tap); the wide epilogue (EW = 4) for the per-tap kernels with one accumulator (the short-K linears / 1x1 convs)
 int launch_gemm2(const GemmLaunch& l, cudaStream_t stream) {
   const int key = l.bn * 1000 + l.nsub * 100 + l.ew * 10 + (l.tr ? 1 : 0);
   switch (key) {
@@ -356,7 +351,6 @@ int launch_gemm2(const GemmLaunch& l, cudaStream_t stream) {
     case 160121: return launch2<160, 1, 2, 1>(l, stream);
     case 192121: return launch2<192, 1, 2, 1>(l, stream);
     case 256121: return launch2<256, 1, 2, 1>(l, stream);
-    case 160221: return launch2<160, 2, 2, 1>(l, stream);
     default: break;
   }
   set_error("no CTA-pair kernel for this BLOCK_N / accumulators / epilogue width / tap reuse combination");

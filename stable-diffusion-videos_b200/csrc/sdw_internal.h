@@ -33,26 +33,6 @@ const char* last_error();
   } while (0)
 
 // ---------------------------------------------------------------------------
-// kernel launch with the programmatic-dependent-launch attribute (SDW_PDL=0 disables it)
-// ---------------------------------------------------------------------------
-bool pdl_enabled();
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                              Args&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
-// ---------------------------------------------------------------------------
 // tcgen05 implicit-GEMM (conv3x3 / conv1x1 / linear / batched matmul)
 // ---------------------------------------------------------------------------
 // out[pix, n] = epi( sum_{tap, c} A[lattice(tap)][pix shifted by (dx,dy)][c] * Wt[n][tap*Cp + c] )
@@ -151,9 +131,9 @@ struct GemmDesc {
   int vt_col0 = 0, vt_d = 0, vt_heads = 0, vt_ntok = 0;
   __half* vt = nullptr;
   int64_t vt_ld = 0;
-  int bn = 0;   // 0 = auto
+  int bn = 0;   // 0 = auto; 192 and 256 need the 2-CTA kernel
   int ver = 0;  // 0 = auto, 1 / 2 force a kernel version
-  int nsub = 0; // 0 = auto, 1 / 2: accumulators per activation tile in the 2-CTA kernel
+  int nsub = 0; // 0 = auto, 1 / 2: accumulators per activation tile in the 2-CTA kernel (2: per-tap mainloop only)
   int ew = 0;   // 0 = auto, 2 / 4: epilogue warps per TMEM lane quarter in the 2-CTA kernel (4 needs the TMA epilogue)
   int tr = 0;   // 0 = auto, 1 = never, 2 = require the tap-reuse mainloop (3x3 stride-1 conv, W % 16 == 0, H % 8 == 0)
   int et = 0;   // 0 = auto, 1 = never, 2 = require the TMA epilogue
@@ -162,7 +142,6 @@ struct GemmDesc {
 int plan_gemm(const GemmDesc& d, GemmLaunch* out);
 int launch_gemm(const GemmLaunch& l, cudaStream_t stream);
 int launch_gemm2(const GemmLaunch& l, cudaStream_t stream);
-int gemm2_init();
 void set_plan_only(bool on);
 int gemm_init();  // resolves the driver entry point, sets smem attributes
 // shared-memory budget of the 2-CTA kernel (sdw_gemm2.cu): barriers, then the operand ring, then the epilogue buffers

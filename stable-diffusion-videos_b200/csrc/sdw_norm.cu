@@ -7,8 +7,6 @@
 #include "sdw_internal.h"
 #include "sdw_ptx.cuh"
 
-#include <cstdlib>
-
 namespace sdw {
 
 // =============================================================================================
@@ -24,15 +22,13 @@ static constexpr int GN_MAX_GROUPS = 64;
 // per-thread partials go to shared memory and are reduced in index order (bit-reproducible).
 __global__ void __launch_bounds__(256) gn_partial_det_kernel(const __half* __restrict__ x, int64_t ld, int C, int G,
                                                              int64_t P, int pix_per_chunk,
-                                                             float2* __restrict__ part, int rev) {
+                                                             float2* __restrict__ part) {
   extern __shared__ float sm[];  // [rows][C] sums then [rows][C] squares
-  pdl_wait();
-  pdl_launch_dependents();
-  // blocks walk the tensor from its END when `rev` is set: the producing GEMM wrote it front to back, so the tail is what
-  // the 126 MB L2 still holds (a front-to-back read of a 157 MB tensor evicts every line just before it is needed); this
-  // pass then ends at the front, which is where gn_apply starts
-  const int b = rev ? static_cast<int>(gridDim.y) - 1 - static_cast<int>(blockIdx.y) : static_cast<int>(blockIdx.y);
-  const int chunk = rev ? static_cast<int>(gridDim.x) - 1 - static_cast<int>(blockIdx.x) : static_cast<int>(blockIdx.x);
+  // blocks walk the tensor from its END: the producing GEMM wrote it front to back, so the tail is what the 126 MB L2
+  // still holds (a front-to-back read of a 157 MB tensor evicts every line just before it is needed); this pass then
+  // ends at the front, which is where gn_apply starts (profiles/r02_norm_reverse_order_ab.txt)
+  const int b = static_cast<int>(gridDim.y) - 1 - static_cast<int>(blockIdx.y);
+  const int chunk = static_cast<int>(gridDim.x) - 1 - static_cast<int>(blockIdx.x);
   const int cg = C / G;
   const int vecs = C / 8;
   const int rows = max(1, min(min(static_cast<int>(blockDim.x) / vecs, 16), 6144 / C));
@@ -98,8 +94,6 @@ __global__ void __launch_bounds__(256) gn_partial_det_kernel(const __half* __res
 // one warp per (b, g): fixed-order reduction of the chunk partials -> (mean, rstd)
 __global__ void __launch_bounds__(256) gn_finalize_kernel(const float2* __restrict__ part, int nchunks, int G, int BG,
                                                           float count, float eps, float2* __restrict__ stats) {
-  pdl_wait();
-  pdl_launch_dependents();
   const int idx = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (idx >= BG) return;
   const int lane = threadIdx.x & 31;
@@ -129,8 +123,6 @@ __global__ void __launch_bounds__(256, 3) gn_apply_kernel(const __half* __restri
   extern __shared__ float gn_aff[];  // [C] sa, [C] sb
   float* sa = gn_aff;
   float* sb = gn_aff + C;
-  pdl_wait();
-  pdl_launch_dependents();
   const int b = blockIdx.y;
   const int cg = C / G;
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
@@ -224,12 +216,6 @@ __global__ void __launch_bounds__(256, 3) gn_apply_kernel(const __half* __restri
 //  the slice normalised while still in L2 — was built, measured slower (64x64x320, batch 32: 130 us vs 82 us; VAE
 //  512x512x128: 2.1 ms vs 0.82 ms: 18 clusters of 8 CTAs keep too few loads in flight) and removed.)
 
-// back-to-front block order of the statistics / LayerNorm passes (L2 reuse of the producer's output); SDW_NORM_REV=0 = A/B
-int norm_reverse() {
-  static const int v = [] { const char* e = std::getenv("SDW_NORM_REV"); return e ? std::atoi(e) : 1; }();
-  return v;
-}
-
 // chunks per sample: enough blocks to fill the machine (B * nchunks >= ~4 waves) while keeping >= 16 pixels each
 int gn_chunks(int64_t P, int B) {
   int64_t want = (148 * 7 + B - 1) / B;  // 7 blocks of the stats kernel fit an SM (30 KB of shared memory each)
@@ -255,18 +241,18 @@ int groupnorm(const __half* x, int64_t ldx, int B, int64_t P, int C, int G, cons
   const size_t smem = static_cast<size_t>(2) * rows * C * sizeof(float);
   SDW_REQUIRE(smem <= 48 * 1024, "GroupNorm: channel count too large for the stats kernel");
   float2* stats = partial_ws + static_cast<size_t>(B) * nchunks * G;
-  SDW_CUDA_OK(launch_pdl(gn_partial_det_kernel, dim3(nchunks, B), dim3(256), smem, stream, x, ldx, C, G, P, ppc, partial_ws,
-                         norm_reverse()));
+  gn_partial_det_kernel<<<dim3(nchunks, B), 256, smem, stream>>>(x, ldx, C, G, P, ppc, partial_ws);
   const int BG = B * G;
-  SDW_CUDA_OK(launch_pdl(gn_finalize_kernel, dim3((BG + 7) / 8), dim3(256), 0, stream, partial_ws, nchunks, G, BG,
-                         static_cast<float>(P) * (C / G), eps, stats));
+  gn_finalize_kernel<<<(BG + 7) / 8, 256, 0, stream>>>(partial_ws, nchunks, G, BG, static_cast<float>(P) * (C / G), eps,
+                                                       stats);
   // one full wave: 148 SMs x 8 resident 256-thread blocks, split evenly over the samples (the former fixed ~100-pixel
   // tiles gave 1376 blocks = 1.16 waves at 64x64x320, batch 32: the second wave ran 16 % full)
   const int64_t per_sample = std::max<int64_t>(1, (148 * 3) / B);  // 3 resident blocks per SM (launch bounds)
   const int ppb = static_cast<int>(std::max<int64_t>(1, (P + per_sample - 1) / per_sample));
   const unsigned tiles = static_cast<unsigned>((P + ppb - 1) / ppb);
-  SDW_CUDA_OK(launch_pdl(gn_apply_kernel, dim3(tiles, B), dim3(256), static_cast<size_t>(2) * C * sizeof(float), stream, x, ldx,
-                         C, G, P, stats, gamma, beta, silu, y, ldy, ppb));
+  gn_apply_kernel<<<dim3(tiles, B), 256, static_cast<size_t>(2) * C * sizeof(float), stream>>>(x, ldx, C, G, P, stats, gamma,
+                                                                                            beta, silu, y, ldy, ppb);
+  SDW_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
@@ -277,12 +263,10 @@ template <int MAXV, int R>  // 16-byte vectors per lane per row, rows per warp (
 __global__ void __launch_bounds__(256) layernorm_kernel(const __half* __restrict__ x, int64_t ldx, int64_t rows,
                                                         int C, const float* __restrict__ gamma,
                                                         const float* __restrict__ beta, float eps,
-                                                        __half* __restrict__ y, int64_t ldy, int rev) {
-  pdl_wait();
-  pdl_launch_dependents();
-  // `rev`: blocks walk the rows from the END — the tail of the tensor is what the L2 still holds of the producing GEMM's
+                                                        __half* __restrict__ y, int64_t ldy) {
+  // blocks walk the rows from the END — the tail of the tensor is what the L2 still holds of the producing GEMM's
   // output, and the consumer GEMM then finds the head of the normalised tensor (written last) in L2
-  const int64_t blk = rev ? static_cast<int64_t>(gridDim.x) - 1 - blockIdx.x : static_cast<int64_t>(blockIdx.x);
+  const int64_t blk = static_cast<int64_t>(gridDim.x) - 1 - blockIdx.x;
   const int64_t row0 = (blk * (blockDim.x >> 5) + (threadIdx.x >> 5)) * R;
   if (row0 >= rows) return;
   const int lane = threadIdx.x & 31;
@@ -366,11 +350,9 @@ template <int LPR, int ITER>
 __global__ void __launch_bounds__(256) layernorm_c40_kernel(const __half* __restrict__ x, int64_t ldx, int64_t rows,
                                                             const float* __restrict__ gamma,
                                                             const float* __restrict__ beta, float eps,
-                                                            __half* __restrict__ y, int64_t ldy, int rev) {
+                                                            __half* __restrict__ y, int64_t ldy) {
   constexpr int C = 40 * LPR, RW = 32 / LPR;  // channels; rows per warp and iteration
   extern __shared__ float ln_gb[];             // [C] gamma, [C] beta
-  pdl_wait();
-  pdl_launch_dependents();
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
     ln_gb[c] = gamma[c];
     ln_gb[C + c] = beta[c];
@@ -378,7 +360,7 @@ __global__ void __launch_bounds__(256) layernorm_c40_kernel(const __half* __rest
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int sub = lane % LPR, rsel = lane / LPR;  // position inside the row's lane group; which of the warp's rows
-  const int64_t blk = rev ? static_cast<int64_t>(gridDim.x) - 1 - blockIdx.x : static_cast<int64_t>(blockIdx.x);
+  const int64_t blk = static_cast<int64_t>(gridDim.x) - 1 - blockIdx.x;  // back to front, as layernorm_kernel
   const int64_t row_base = (blk * (blockDim.x >> 5) + warp) * (RW * ITER);
   uint4 u[ITER][5];
 #pragma unroll
@@ -447,12 +429,12 @@ __global__ void __launch_bounds__(256) layernorm_c40_kernel(const __half* __rest
 
 template <int LPR>
 static int launch_ln_c40(const __half* x, int64_t ldx, int64_t rows, const float* gamma, const float* beta, float eps,
-                         __half* y, int64_t ldy, int rev, cudaStream_t stream) {
+                         __half* y, int64_t ldy, cudaStream_t stream) {
   constexpr int ITER = 2, C = 40 * LPR;
   const int64_t rows_per_block = 8 * (32 / LPR) * ITER;
   const unsigned blocks = static_cast<unsigned>((rows + rows_per_block - 1) / rows_per_block);
-  SDW_CUDA_OK(launch_pdl(layernorm_c40_kernel<LPR, ITER>, dim3(blocks), dim3(256), static_cast<size_t>(2) * C * sizeof(float),
-                         stream, x, ldx, rows, gamma, beta, eps, y, ldy, rev));
+  layernorm_c40_kernel<LPR, ITER><<<blocks, 256, static_cast<size_t>(2) * C * sizeof(float), stream>>>(x, ldx, rows, gamma,
+                                                                                                      beta, eps, y, ldy);
   SDW_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -461,25 +443,23 @@ int layernorm(const __half* x, int64_t ldx, int64_t rows, int C, const float* ga
               __half* y, int64_t ldy, cudaStream_t stream) {
   SDW_REQUIRE(C % 8 == 0 && C <= 8 * 32 * 8, "LayerNorm: C % 8 == 0 and C <= 2048");
   const int vecs = C / 8;
-  const int rev = norm_reverse();
-  // the UNet widths take the lane-group kernel; SDW_LN_C40=0 keeps the generic one (A/B)
-  static const int c40_env = [] { const char* e = std::getenv("SDW_LN_C40"); return e ? std::atoi(e) : 1; }();
+  // the UNet widths take the lane-group kernel
   const bool vec_ok = (ldx % 8 == 0) && (ldy % 8 == 0) && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) == 0 &&
                       ((reinterpret_cast<uintptr_t>(gamma) | reinterpret_cast<uintptr_t>(beta)) & 15) == 0;
-  if (c40_env && vec_ok) {
-    if (C == 320) return launch_ln_c40<8>(x, ldx, rows, gamma, beta, eps, y, ldy, rev, stream);
-    if (C == 640) return launch_ln_c40<16>(x, ldx, rows, gamma, beta, eps, y, ldy, rev, stream);
-    if (C == 1280) return launch_ln_c40<32>(x, ldx, rows, gamma, beta, eps, y, ldy, rev, stream);
+  if (vec_ok) {
+    if (C == 320) return launch_ln_c40<8>(x, ldx, rows, gamma, beta, eps, y, ldy, stream);
+    if (C == 640) return launch_ln_c40<16>(x, ldx, rows, gamma, beta, eps, y, ldy, stream);
+    if (C == 1280) return launch_ln_c40<32>(x, ldx, rows, gamma, beta, eps, y, ldy, stream);
   }
   if (vecs <= 64) {
     const unsigned blocks = static_cast<unsigned>((rows + 31) / 32);
-    SDW_CUDA_OK(launch_pdl(layernorm_kernel<2, 4>, dim3(blocks), dim3(256), 0, stream, x, ldx, rows, C, gamma, beta, eps, y, ldy, rev));
+    layernorm_kernel<2, 4><<<blocks, 256, 0, stream>>>(x, ldx, rows, C, gamma, beta, eps, y, ldy);
   } else if (vecs <= 160) {
     const unsigned blocks = static_cast<unsigned>((rows + 15) / 16);
-    SDW_CUDA_OK(launch_pdl(layernorm_kernel<5, 2>, dim3(blocks), dim3(256), 0, stream, x, ldx, rows, C, gamma, beta, eps, y, ldy, rev));
+    layernorm_kernel<5, 2><<<blocks, 256, 0, stream>>>(x, ldx, rows, C, gamma, beta, eps, y, ldy);
   } else {
     const unsigned blocks = static_cast<unsigned>((rows + 7) / 8);
-    SDW_CUDA_OK(launch_pdl(layernorm_kernel<8, 1>, dim3(blocks), dim3(256), 0, stream, x, ldx, rows, C, gamma, beta, eps, y, ldy, rev));
+    layernorm_kernel<8, 1><<<blocks, 256, 0, stream>>>(x, ldx, rows, C, gamma, beta, eps, y, ldy);
   }
   SDW_CUDA_OK(cudaGetLastError());
   return 0;
@@ -573,8 +553,6 @@ __global__ void __launch_bounds__(512) conv_in_kernel(const TIn* __restrict__ x,
   const int64_t P = static_cast<int64_t>(B) * H * W;
   const int64_t p0 = static_cast<int64_t>(blockIdx.x) * pix_per_block;
   const int np = static_cast<int>(min(static_cast<int64_t>(pix_per_block), P - p0));
-  pdl_wait();
-  pdl_launch_dependents();
   for (int i = threadIdx.x; i < pix_per_block * KP; i += blockDim.x) {
     const int k = i % KP;
     const int c = k % CIN;
@@ -697,8 +675,6 @@ __global__ void __launch_bounds__(256) conv_out_kernel(const __half* __restrict_
       }
     }
   }
-  pdl_wait();
-  pdl_launch_dependents();
   const int c8n = C / 8;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
   const int tx = tile % tiles_x, ty = (tile / tiles_x) % tiles_y;

@@ -287,14 +287,6 @@ __host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N) {
 }
 
 // ----------------------------------------------------------------------------
-// programmatic dependent launch: a kernel launched with the PDL attribute may start while its predecessor drains;
-// everything before pdl_wait() (barrier init, TMEM alloc, descriptor prefetch) overlaps the predecessor's tail,
-// nothing after it runs until the predecessor grid has completed and its writes are visible.
-// ----------------------------------------------------------------------------
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-// ----------------------------------------------------------------------------
 // small math helpers
 // ----------------------------------------------------------------------------
 __device__ __forceinline__ float silu_f(float x) { return x / (1.f + __expf(-x)); }

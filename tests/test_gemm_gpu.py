@@ -312,8 +312,7 @@ def test_gemm_2cta_two_accumulators(B, H, W, Cc, N, conv):
 
 
 # ---- tap reuse: one 10-row activation box per (channel chunk, kx) feeds the three ky taps of a 3x3 stride-1 conv ---------
-@pytest.mark.parametrize("B,H,W,Cc,N,bn,nsub", [(4, 64, 64, 320, 320, 160, 1), (4, 64, 64, 320, 320, 160, 2),
-                                                 (2, 32, 32, 640, 640, 256, 1), (2, 16, 16, 128, 1280, 256, 1),
+@pytest.mark.parametrize("B,H,W,Cc,N,bn,nsub", [(4, 64, 64, 320, 320, 160, 1), (2, 32, 32, 640, 640, 256, 1), (2, 16, 16, 128, 1280, 256, 1),
                                                  (3, 16, 16, 64, 480, 128, 1), (1, 8, 16, 72, 200, 192, 1),
                                                  (1, 128, 128, 128, 128, 128, 1), (1, 24, 48, 104, 320, 0, 0)])
 def test_gemm_conv3x3_tap_reuse(B, H, W, Cc, N, bn, nsub):

@@ -93,6 +93,10 @@ def test_opt_in_variants_are_refused_outside_their_domain(native):
         _plan(native, 32, 8, 8, 1280, 1280, 1, tr=2)          # tap reuse needs W % 16 == 0
     with pytest.raises(native.SdwError):
         _plan(native, 32, 64, 64, 320, 320, 1, ew=4)           # the 16-warp epilogue belongs to the per-tap kernels
+    with pytest.raises(native.SdwError):
+        _plan(native, 32, 64, 64, 320, 320, 1, nsub=2, tr=2)   # two accumulators need the per-tap mainloop
+    with pytest.raises(native.SdwError):
+        _plan(native, 1, 1, 4096, 320, 320, 0, ver=1, bn=256)  # BLOCK_N 256 is a CTA-pair tile
     p = _plan(native, 1, 1, 131072, 320, 2560, 0, mode=1, resid=False, ew=4)
     assert p["ew"] == 4 and p["epi_tma"] == 1 and p["grid"] == 148, p
     p = _plan(native, 1, 1, 131072, 320, 2560, 0, mode=1, resid=False)      # short K: chosen automatically

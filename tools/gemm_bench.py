@@ -61,8 +61,10 @@ if __name__ == "__main__":
             variants = ((0, 0, 0), (160, 1, 1), (256, 1, 1))
             if conv and W % 16 == 0 and H % 8 == 0:  # tr: 1 = per-tap activation tiles, 2 = tap-reuse mainloop
                 variants = ((0, 0, 0), (0, 0, 1), (128, 1, 1), (128, 1, 2), (160, 1, 1), (160, 1, 2), (192, 1, 2),
-                            (256, 1, 1), (256, 1, 2), (160, 2, 1), (160, 2, 2))
+                            (256, 1, 1), (256, 1, 2), (160, 2, 1))
             for bn, nsub, tr in variants:
+                if ver == 1 and (bn in (192, 256) or tr == 2):  # CTA-pair-only tiles
+                    continue
                 for epi in (True,):
                     ms, tf = bench(B, H, W, C, N, conv, bn=bn, ver=ver, epi=epi, nsub=nsub, tr=tr)
                     print(f"{name:36s} B={B:3d} v{ver} bn={bn or 'auto':>4} nsub={nsub} tr={tr} "
